@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """SAC gradient steps/s on B200 (BASELINE.json metric), with roofline, CPU baseline, e2e and the other BASELINE configs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload LL|VS|MS|C10|C10O] [--replicas R]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload LL|VS|MS|C10|C10O] [--replicas R] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's CPU learner path on the host cores
 
@@ -10,9 +10,17 @@ learner replica on the GPU.
 
 `value`  learner-steps/s with the replay ring resident in HBM: index sampling + gather + step all on the device, CUDA
          graphs of 8/4/2/1 steps.  Every graph is instantiated BEFORE the clock starts (b200sac_prepare) and >= 16 warm-up
-         steps run first.  The timed region is a train of back-to-back windows of EXACTLY K steps each, a CUDA event between
-         windows, barrier + synchronize on both sides of the train; `ms_per_step` is the MEDIAN window (per window: max over
-         ranks), so a K = 20 run is as steady as a K = 2000 one; all window statistics and per-rank medians are in `timing`.
+         steps run first.  The timed region is EXACTLY K steps, run as a train of back-to-back windows (multiples of 8 steps,
+         so each window is whole 8-step graphs), a CUDA event between windows, barrier + synchronize on both sides of the
+         train; `ms_per_step` is the MEDIAN over windows of the window's time per step (per window: max over ranks); all
+         window statistics and per-rank medians are in `timing`.
+         --dump-outputs DIR writes what the timed region computed in its last step (rank 0): the losses of every replica and
+         each replica's parameters, target networks and Adam moments, as DIR/<name>.npy (float32; Adam step counts and the
+         GEMM back-end used, `precision`, float64).  Inputs are seeded, so the same arguments give the same inputs on every
+         run; pin --precision 0 or 1 to compare dumps, since the default -1 picks the back-end by a timing probe.  Above
+         64 MB in all, every large tensor is replaced by a fixed seeded sample of its elements (flattened).  The library
+         must have been built (__graft_entry__.build()) from the sources in the tree: the benchmark refuses a missing or
+         stale one, and compiles nothing and writes nothing in the source tree.
 `e2e`    the same metric through the reference-shaped `Learner.update()` with the replay ring in pinned HOST memory: per
          step a host-side sample + gather, an H2D copy of the minibatch and a D2H read of the losses, synchronously --
          the reference's update() contract.
@@ -31,7 +39,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree untouched (it may be read-only)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 # ring sizes, declared once: `value` samples the device ring (BASELINE config 2: 1M transitions resident in HBM);
@@ -343,6 +353,36 @@ def make_learner(workload, cfg_path, device_index, buffer_size, precision=1):
     return L.MTSACLearner(None, None, cfg_path, write_mode=False, server=srv, device_index=device_index, precision=precision)
 
 
+DUMP_BYTES = 60 << 20        # array payload; with the .npy headers the dump stays under 64 MB
+
+
+def dump_outputs(core, out_dir):
+    """The state the last step left, as a caller reads it back (read_losses, get_named, get_steps), to out_dir/<name>.npy:
+    `losses` [R][4] (critic, actor, alpha, entropy), `param.<tensor>` / `adam_m.<tensor>` / `adam_v.<tensor>` [R][shape] for
+    every tensor of the layout (targets included), `adam_steps` [R][n] and `precision` [1] (the GEMM back-end that computed
+    them: 0 = fp32 FFMA, 1 = 3xTF32 tcgen05).  If the arrays exceed DUMP_BYTES, each one of more
+    than 4096 elements is replaced by the same fraction of its (flattened) elements at indices drawn with a fixed seed."""
+    from distributed_sac_b200 import _lib
+    R = core.cfg.replicas
+    arrays = {"losses": core.read_losses(1)[0].numpy()}
+    for tag, which in (("param", _lib.PARAMS), ("adam_m", _lib.ADAM_M), ("adam_v", _lib.ADAM_V)):
+        per_replica = [core.get_named(which, r) for r in range(R)]
+        for name in per_replica[0]:
+            arrays[f"{tag}.{name}"] = np.stack([p[name].numpy() for p in per_replica])
+    arrays["adam_steps"] = np.array([core.get_steps(r) for r in range(R)], dtype=np.float64)
+    arrays["precision"] = np.array([core.cfg.precision], dtype=np.float64)
+    big = sum(a.nbytes for a in arrays.values() if a.size > 4096)
+    small = sum(a.nbytes for a in arrays.values()) - big
+    frac = min(1.0, (DUMP_BYTES - small) / max(big, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0 and a.size > 4096:
+            flat = a.reshape(-1)
+            idx = np.random.default_rng(0).choice(flat.size, max(1, int(flat.size * frac)), replace=False)
+            a = flat[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class Bench:
     def __init__(self, args):
         self.args = args
@@ -374,9 +414,12 @@ class Bench:
         return torch.stack(out).cpu()
 
     # ---- the timing protocol ------------------------------------------------------------------------------------
-    def timed_windows(self, core, ring, K, W, target_steps, clocks=None):
-        """Train of n windows of exactly K steps; returns (median window ms [max over ranks per window], info)."""
-        n = max(3, min(400, math.ceil(target_steps / K)))
+    def timed_windows(self, core, ring, steps, W, clocks=None):
+        """Train of back-to-back windows that together run exactly `steps` steps; returns (median over windows of the window's
+        ms per step [max over ranks per window], info)."""
+        w = 8 * max(1, math.ceil(steps / 128))           # ~16 windows, each whole 8-step graphs but (maybe) the last
+        sizes = [w] * (steps // w) + ([steps % w] if steps % w else [])
+        n = len(sizes)
         warm = max(W, 16)
         with torch.cuda.stream(self.stream):
             core.prepare(ring)                            # every graph instantiated before the clock starts
@@ -386,8 +429,8 @@ class Bench:
             if clocks:
                 clocks.mark_begin()
             evs[0].record()
-            for i in range(n):
-                core.step_sampled(ring, K)
+            for i, k in enumerate(sizes):
+                core.step_sampled(ring, k)
                 evs[i + 1].record()
             self.barrier()
             if clocks:
@@ -395,15 +438,18 @@ class Bench:
         ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(n)]
         allr = self.gather_ranks(ms)                      # [world][n]
         per_window = allr.max(dim=0).values               # max over ranks, per window
-        med = float(per_window.median())
-        info = {"windows": n, "steps_per_window": K, "warmup_steps": warm,
-                "window_ms": {"min": float(per_window.min()), "median": med, "max": float(per_window.max()), "first": float(per_window[0])},
-                "per_rank_median_window_ms": [float(x) for x in allr.median(dim=1).values],
+        per_step = per_window / torch.tensor(sizes, dtype=per_window.dtype)
+        med = float(per_step.median())
+        info = {"windows": n, "timed_steps": steps, "steps_per_window": sizes, "warmup_steps": warm,
+                "window_ms": {"min": float(per_window.min()), "median": float(per_window.median()), "max": float(per_window.max()),
+                              "first": float(per_window[0])},
+                "step_ms": {"min": float(per_step.min()), "median": med, "max": float(per_step.max()), "first": float(per_step[0])},
+                "per_rank_median_step_ms": [float(x) for x in (allr / torch.tensor(sizes, dtype=allr.dtype)).median(dim=1).values],
                 "train_ms": float(allr.sum(dim=1).max()),
-                "rule": "ms_per_step = median over windows of (max over ranks of the window's device time) / K"}
+                "rule": "ms_per_step = median over windows of (max over ranks of the window's device time) / (the window's steps)"}
         return med, info
 
-    def gpu_leg(self, workload, R, precision, K, W, target_steps, ring_n, seed0=1234, detail=False, clocks=None, bcast=False):
+    def gpu_leg(self, workload, R, precision, steps, W, ring_n, seed0=1234, detail=False, clocks=None, bcast=False, dump=None):
         from distributed_sac_b200.core import Replay, SacCore
         from distributed_sac_b200.replicas import broadcast_initial_params
         core = SacCore(core_config(workload, R, precision), self.local, seed=seed0 + self.rank)
@@ -411,16 +457,18 @@ class Bench:
             broadcast_initial_params(core, src=0)         # independent replicas: ONE collective (SURVEY 8(e))
         ring = Replay(core, ring_n, where="device", seed=99 + self.rank)
         ring.fill_synthetic(ring_n, seed=seed0 + self.rank)
-        ms, info = self.timed_windows(core, ring, K, W, target_steps, clocks)
-        losses = core.read_losses(min(K, 64))
+        ms, info = self.timed_windows(core, ring, steps, W, clocks)
+        losses = core.read_losses(min(steps, 64))
         assert torch.isfinite(losses).all(), f"non-finite losses in the timed region ({workload})"
+        if dump:                                          # before the detail runs below step the core further
+            dump_outputs(core, dump)
         total = self.gather_ranks([float(R)]).sum().item()                 # learners over all ranks
-        out = {"value": total * K / (ms * 1e-3), "ms_per_step": ms / K, "learners": int(total), "timing": info,
+        out = {"value": total / (ms * 1e-3), "ms_per_step": ms, "learners": int(total), "timing": info,
                "launches_per_step": core.launches_per_step + 1,
                "gemm_backend": ("layer-chained fp32 FFMA (chain.cuh)" if (precision == 0 and workload == "LL") else
                                 "fp32 FFMA" if precision == 0 else "tcgen05 3xTF32")}
         work = WORK[workload]
-        step_s = ms * 1e-3 / K
+        step_s = ms * 1e-3
         out["hbm_frac"] = R * work["mbytes"] * 1e6 / step_s / 1e9 / self.pk["hbm"]
         out["tensor_frac"] = R * work["gflop"] * 1e9 / step_s / 1e12 / self.pk["tf"]
         if detail:
@@ -562,7 +610,12 @@ def main():
                     help="0 = fp32 FFMA (layer-chained kernels for LL-class shapes), 1 = 3xTF32 tcgen05 GEMMs, -1 = probe both, headline = faster")
     ap.add_argument("--configs", default="auto", help="'auto' = short legs of VS, MS, C10 + config 4 placement + learners-per-GPU sweep; 'none' = headline only")
     ap.add_argument("--sweep", default="4,16,64", help="learners-per-GPU values of the sweep (headline workload, short legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's losses, parameters and Adam state as DIR/<name>.npy "
+                         "(pin --precision when comparing dumps: -1 picks the back-end by timing)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -570,7 +623,11 @@ def main():
         return run_reference(args, rank, world)
 
     import __graft_entry__ as ge
-    ge.build()
+    if ge.library_is_stale():
+        raise SystemExit(f"{ge.LIB} is missing or older than its sources: build it with "
+                         "`python -c 'import __graft_entry__ as g; g.build()'` (the benchmark compiles nothing)")
+    from distributed_sac_b200 import _lib
+    _lib.load()
     from distributed_sac_b200.replicas import shard_replicas
 
     if not torch.cuda.is_available():
@@ -597,11 +654,12 @@ def main():
     cands = [0, 1] if args.precision < 0 else [args.precision]
     if len(cands) > 1:            # short probe of both back-ends; the full timed run uses the faster one
         for pr in cands:
-            leg = b.gpu_leg(wl, R, pr, 100, 16, 600, 1 << 16)
+            leg = b.gpu_leg(wl, R, pr, 600, 16, 1 << 16)
             by_precision["probe"]["fp32" if pr == 0 else "tc3xtf32"] = leg["value"]
         args.precision = 0 if by_precision["probe"]["fp32"] >= by_precision["probe"]["tc3xtf32"] else 1
     log("back-end probe")
-    head = b.gpu_leg(wl, R, args.precision, K, W, 8000 if wl == "LL" else 2000, args.ring, detail=True, clocks=clocks, bcast=True)
+    head = b.gpu_leg(wl, R, args.precision, K, W, args.ring, detail=True, clocks=clocks, bcast=True,
+                     dump=args.dump_outputs if b.rank == 0 else None)
     clk = clocks.stop()
     by_precision["final"]["fp32" if args.precision == 0 else "tc3xtf32"] = head["value"]
     row_bytes = 4 * ((2 * core_config(wl, 1).obs_dim + core_config(wl, 1).act_dim + 2 + 31) // 32 * 32)
@@ -627,28 +685,28 @@ def main():
     configs, sweep = {}, {}
     if args.configs == "auto":
         for w2 in [w for w in ("VS", "MS", "C10") if w != wl]:
-            leg = b.gpu_leg(w2, 1, 1, 50, 16, 400, 1 << 17)
+            leg = b.gpu_leg(w2, 1, 1, 400, 16, 1 << 17)
             e2 = b.e2e_leg(w2, 1, 200, 16)
             configs[w2] = {"workload": WORKLOAD_DESC[w2], "value": leg["value"], "unit": "steps/s", "ms_per_step": leg["ms_per_step"],
                            "n_gpus": world, "learners": leg["learners"], "e2e": {k: e2[k] for k in ("value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step", "steps")},
                            "roofline": {"hbm_frac": leg["hbm_frac"], "tensor_frac": leg["tensor_frac"],
                                         "algorithmic_bytes_per_step": WORK[w2]["mbytes"] * 1e6, "algorithmic_flop_per_step": WORK[w2]["gflop"] * 1e9},
-                           "gemm_backend": leg["gemm_backend"], "launches_per_step": leg["launches_per_step"], "timing": leg["timing"]["window_ms"]}
+                           "gemm_backend": leg["gemm_backend"], "launches_per_step": leg["launches_per_step"], "timing": leg["timing"]["step_ms"]}
             log(f"config leg {w2}")
         # BASELINE config 4: 10 independent MTSAC learners over the GPUs of this run (8 GPUs: 2,2,1,1,1,1,1,1)
         place = shard_replicas(10, world)
         mine = len(place[b.rank])
-        leg = b.gpu_leg("MS", max(mine, 1), 1, 50, 16, 300, 1 << 16)
+        leg = b.gpu_leg("MS", max(mine, 1), 1, 300, 16, 1 << 16)
         configs["cfg4_10_learners"] = {"workload": "10 independent " + WORKLOAD_DESC["MS"] + " replicas, no gradient all-reduce",
                                        "placement_learners_per_gpu": [len(p) for p in place], "value": leg["value"], "unit": "steps/s (sum over the 10 learners)",
                                        "ms_per_step": leg["ms_per_step"], "n_gpus": world, "learners": leg["learners"],
                                        "roofline": {"hbm_frac_of_rank0": leg["hbm_frac"], "tensor_frac_of_rank0": leg["tensor_frac"]},
-                                       "timing": leg["timing"]["window_ms"]}
+                                       "timing": leg["timing"]["step_ms"]}
         log("config 4 placement")
         for r_extra in [int(x) for x in args.sweep.split(",") if x]:
             sweep[str(r_extra)] = {}
             for pr in (0, 1):
-                leg = b.gpu_leg(wl, r_extra, pr, 50, 16, 200, max(1 << 14, (1 << 19) // r_extra), seed0=77)
+                leg = b.gpu_leg(wl, r_extra, pr, 200, 16, max(1 << 14, (1 << 19) // r_extra), seed0=77)
                 sweep[str(r_extra)]["fp32" if pr == 0 else "tc3xtf32"] = {"value": leg["value"], "hbm_frac": leg["hbm_frac"]}
 
     log("learners-per-GPU sweep")
