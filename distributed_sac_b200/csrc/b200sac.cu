@@ -1404,7 +1404,7 @@ static int build_plan(b200sac* h) {
     const int cols = wide ? kHb4Cols : kHbCols;
     l.grid = dim3(((P.Kdim + cols - 1) / cols) * ((B + rows_per - 1) / rows_per), P.nets, R);
     l.block = dim3(256);
-    l.smem = ((size_t)rows_per * P.NO + (wide ? 1024 : 256) * (size_t)P.NO) * sizeof(float);
+    l.smem = ((size_t)pad4((int64_t)rows_per * P.NO) + (wide ? 1024 : 256) * (size_t)P.NO) * sizeof(float);   // (head_bwd4 aligns its reduction tiles)
     h->plan.push_back(l);
   };
   // ---- Phase C: critic backward + Adam/Polyak ----------------------------------------------

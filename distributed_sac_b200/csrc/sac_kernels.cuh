@@ -715,7 +715,8 @@ __global__ void __launch_bounds__(256) head_bwd4_kernel(StepConst K, HeadBwdArgs
   const int M = r1 - r0;
   if (M <= 0) return;
   float* sd = sm;                                   // [M][NO]
-  float* red = sm + (size_t)rows_per * NO;          // [16 row groups][16 col quads][NO][4]
+  // [16 row groups][16 col quads][NO][4], stored as float4: 16-B aligned behind sd whatever rows_per * NO is (an odd batch)
+  float* red = sm + (((size_t)rows_per * NO + 3) & ~(size_t)3);
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
 
   if (P.policy_mode) {
